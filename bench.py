@@ -4,6 +4,11 @@
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        # the reference's CPU path (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR      # also write what the last timed step computed (dump_outputs)
+
+--steps is the number of timed steps of the headline loop (`value`, `ms_per_step`, `gpu_launches`); --dump-outputs
+writes what the last of them computed.  The end-to-end loops in `e2e` run their own step counts (bounded so that
+their pipelines fill), reported beside their figures.
 
 One "step" = one pass of the tool-node hot path (decode -> ToolNodeDef.run -> _publish_action ->
 encode -> route) over one batch of `--events` synthetic 1 KB-class agent events per GPU
@@ -29,6 +34,9 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+# the benchmark writes nothing into the tree it runs from (it may be read-only): no bytecode caches (spawned worker
+# processes run this line too, before they import anything from the tree)
+sys.dont_write_bytecode = True
 sys.path.insert(0, os.path.join(ROOT, "calfkit-sdk_b200"))
 sys.path.insert(0, ROOT)
 
@@ -199,6 +207,54 @@ class ClockSampler(threading.Thread):
                 "samples": len(s)}
 
 
+def dump_outputs(out_dir: str, eng, max_records: int = 4096, max_payload_bytes: int = 8 << 20, seed: int = 0) -> None:
+    """Writes what the engine's last plan hands a caller (the payload table, the publish table and the decode columns
+    that BatchEngine.fetch returns) as float .npy files under `out_dir`, so that two builds run with the same arguments
+    can be compared output for output.  The whole batch enters through exact totals and CRC-32s (float64); the rest is
+    a fixed, seeded sample of records and payloads: at most 4096 records and 8 MB of payload bytes (~40 MB of files).
+
+      totals          [records, payloads, live publishes, payload bytes, CRC-32 of the live publishes (fields and
+                       payload bytes, in table order), CRC-32 of the STATUS and ACTION columns of every record]
+      records         sampled record indices
+      columns         the decode columns (calfkit.engine._lib.COLS) of the sampled records, [NUM_COLS, records]
+      publishes       the live publishes of the sampled records, one row each: payload, topic_id, topic_off,
+                      topic_len, record, has_key, partition, payload length
+      payload_index   sampled payload indices;  payload_len: their lengths;  payloads: their bytes, concatenated
+    """
+    import zlib
+    import numpy as np
+    from calfkit.engine._lib import COL
+    out, off, ln, pubs = eng._fetch()
+    cols = eng.columns()
+    n, npay = cols.shape[1], len(ln)
+    fields = ["payload", "topic_id", "topic_off", "topic_len", "record", "has_key", "partition"]
+    live = pubs[pubs["payload"] != 0xFFFFFFFF]
+    table = np.stack([live[f].astype(np.int64) for f in fields], axis=1) if len(live) else np.zeros((0, len(fields)), np.int64)
+    mv = memoryview(out)
+    pub_crc = zlib.crc32(table.tobytes())
+    for p in live["payload"].tolist():                      # payloads are padded in the buffer: CRC the bytes a caller sees
+        pub_crc = zlib.crc32(mv[int(off[p]):int(off[p]) + int(ln[p])], pub_crc)
+    col_crc = zlib.crc32(np.ascontiguousarray(cols[[COL["STATUS"], COL["ACTION"]]]).tobytes())
+
+    rng = np.random.default_rng(seed)
+    recs = np.sort(rng.permutation(n)[:max_records])
+    rows = table[np.isin(table[:, 4], recs)]
+    take = rng.permutation(npay)[:max_records]
+    take = np.sort(take[np.cumsum(ln[take].astype(np.int64)) <= max_payload_bytes])
+    arrays = {
+        "totals": np.array([n, npay, len(live), ln.astype(np.int64).sum(), pub_crc, col_crc], dtype=np.float64),
+        "records": recs.astype(np.float64),
+        "columns": cols[:, recs].astype(np.float64),
+        "publishes": np.concatenate([rows, ln[rows[:, 0]].astype(np.int64)[:, None]], axis=1).astype(np.float64),
+        "payload_index": take.astype(np.float64),
+        "payload_len": ln[take].astype(np.float64),
+        "payloads": np.concatenate([out[int(off[p]):int(off[p]) + int(ln[p])] for p in take] or [np.zeros(0, np.uint8)]).astype(np.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 class CudaArray:
     """wraps a raw device pointer for torch.as_tensor via __cuda_array_interface__"""
     def __init__(self, ptr: int, shape, typestr: str):
@@ -314,6 +370,8 @@ def run_fanout(args, rank, world, local_rank, dev, real_stdout, all_cpus=None) -
     eng.profile(False)
     out_bytes, npay, npub = eng.out_size()
     value = world * n / (ms_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
     # end to end: pinned host in -> device -> pinned host out
     h_in = torch.from_numpy(batch.data.copy()).pin_memory()
     h_off = torch.from_numpy(batch.offsets.copy()).pin_memory()
@@ -462,6 +520,8 @@ def run_reply(args, rank, world, local_rank, dev, real_stdout, all_cpus=None) ->
     eng.profile(False)
     out_bytes, npay, _npub = eng.out_size()
     value = world * n / (ms_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
     h_in = torch.from_numpy(batch.data.copy()).pin_memory()
     h_off = torch.from_numpy(batch.offsets.copy()).pin_memory()
     h_out = torch.empty(out_bytes + (1 << 20), dtype=torch.uint8).pin_memory()
@@ -582,6 +642,8 @@ def run_mixed(args, rank, world, local_rank, dev, real_stdout, all_cpus=None) ->
     eng.profile(False)
     out_bytes, npay, npub = eng.out_size()
     value = world * n / (ms_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
     from calfkit.engine.lane import Arena, LanePipeline
     pipe = LanePipeline(local_rank, lambda e_: (e_.register_topics(topics, num_partitions=NUM_PARTITIONS),
                                                 e_.set_tool_node("tool.get_weather.output", ToolTemplate.from_format(TOOL_FMT)), e_.set_bucketing(True)),
@@ -670,7 +732,11 @@ def main() -> None:
     ap.add_argument("--workload", default="tool_event_1k", choices=["tool_event_1k", "fanout", "reply", "mixed"],
                     help="tool_event_1k = BASELINE.json configs[1] (the headline); fanout = configs[2]: 1 Agent -> 64 tools")
     ap.add_argument("--fanout", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -878,6 +944,10 @@ def main() -> None:
     ms_total = float(t.item())
     ms_step = ms_total / args.steps
     value = world * n / (ms_step / 1e3)
+    if args.dump_outputs:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, lanes[(args.steps - 1) % len(lanes)].eng)    # before the end-to-end loops reuse the lanes
+        barrier()           # the other ranks wait here rather than inside the exchange of the next loop
 
     # ---- end to end (host buffers), pipelined over several engines (3 at N = 1, 2 at N > 1) -----------------
     # step k: lane k%2 takes the batch from pinned host memory (H2D + all kernels, asynchronous) while the
