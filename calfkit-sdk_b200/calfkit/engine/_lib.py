@@ -30,7 +30,7 @@ COLS = ["STATUS", "ACTION", "ERR", "CORR_OFF", "CORR_LEN", "NFRAMES", "FRAMES_OF
 COL = {name: i for i, name in enumerate(COLS)}
 NUM_COLS = len(COLS)
 
-KERNELS = ["walk", "plan", "scan", "emit", "route", "fanout", "canon", "walk_long", "walk_elems"]
+KERNELS = ["walk", "plan", "scan", "emit", "route", "fanout", "canon", "walk_long", "walk_elems", "codec"]
 NUM_KERNELS = len(KERNELS)
 
 PUB_DTYPE = np.dtype([("payload", "<u4"), ("topic_id", "<i4"), ("topic_off", "<u4"), ("topic_len", "<u4"),
@@ -42,7 +42,7 @@ EXPORTS = ["ck_create", "ck_destroy", "ck_last_error", "ck_version", "ck_registe
            "ck_device_buffers", "ck_device_buffers2", "ck_gather_spans", "ck_profile", "ck_profile_read", "ck_fetch_cols",
            "ck_host_alloc", "ck_host_free", "ck_canon_stats", "ck_fetch_output_async",
            "ck_fetch_cols_async", "ck_gate_create", "ck_gate_register", "ck_gate_arrive", "ck_gate_stats", "ck_gate_reset", "ck_submit_recordbatch",
-           "ck_fetch_rb_index", "ck_encode_recordbatch", "ck_group_publishes", "ck_fetch_groups", "ck_comm_create", "ck_comm_connect", "ck_exchange_send", "ck_recv_info", "ck_fetch_received", "ck_peek_received", "ck_fetch_received_async", "ck_set_option"]
+           "ck_fetch_rb_index", "ck_fetch_rb_decompressed", "ck_encode_recordbatch", "ck_group_publishes", "ck_fetch_groups", "ck_comm_create", "ck_comm_connect", "ck_exchange_send", "ck_recv_info", "ck_fetch_received", "ck_peek_received", "ck_fetch_received_async", "ck_set_option"]
 
 _lib = None
 
@@ -102,6 +102,7 @@ def load() -> C.CDLL:
         "ck_fetch_groups": (C.c_int, [vp, u32p, u32p, C.c_int]),
         "ck_submit_recordbatch": (C.c_int, [vp, u8p, C.c_uint64, C.POINTER(C.c_uint32)]),
         "ck_fetch_rb_index": (C.c_int, [vp, i64p, u32p, i64p, i32p, i64p, i32p, u32p]),
+        "ck_fetch_rb_decompressed": (C.c_int, [vp, u8p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "ck_encode_recordbatch": (C.c_int, [vp, u32p, C.c_uint32, C.c_int64, C.c_int64, u8p, C.c_uint64, C.POINTER(C.c_uint64)]),
         "ck_gate_create": (C.c_int, [vp, C.c_uint32, C.c_uint32, C.c_uint64]),
         "ck_gate_register": (C.c_int, [vp, C.c_uint32]),

@@ -74,6 +74,32 @@ class _SpanOffsets:
         return len(self.off) + 1
 
 
+class _RecordBatchBytes:
+    """The byte space the offsets of `BatchEngine.rb_index()` index: the submitted buffer, followed at `base` by the
+    decompressed records sections of its gzip / LZ4 frames.  Those sections are copied from the device once, on the
+    first read that lands in them; a fetch whose host side reads only uncompressed records never copies them."""
+    def __init__(self, engine: "BatchEngine", buf: np.ndarray, base: int):
+        self.engine, self.buf, self.base = engine, buf, base
+        self._submit_no = engine._submit_no
+        self._dec: np.ndarray | None = None
+
+    def decompressed(self) -> np.ndarray:
+        if self._dec is None:
+            if self.engine._submit_no != self._submit_no:
+                raise EngineError("the decompressed records of this fetch were overwritten by a later submit: "
+                                  "read them before submitting the next batch")
+            self._dec = self.engine.rb_decompressed()
+        return self._dec
+
+    def __getitem__(self, s: slice) -> np.ndarray:
+        start, stop = int(s.start), int(s.stop)
+        if stop <= len(self.buf):
+            return self.buf[start:stop]
+        if start >= self.base:
+            return self.decompressed()[start - self.base:stop - self.base]
+        raise IndexError(f"span [{start}, {stop}) straddles the submitted and the decompressed bytes")
+
+
 class BatchOutput:
     """Result of one plan+emit: unique payloads + the publish table that references them."""
 
@@ -177,6 +203,7 @@ class BatchEngine:
         self.num_partitions = 0
         self.n = 0
         self._in_data = self._in_off = None
+        self._submit_no = 0                 # counts submits: the device input buffer a host view refers to is still current
 
     # ------------------------------------------------------------------------------------------
     def close(self) -> None:
@@ -286,24 +313,48 @@ class BatchEngine:
         """H2D + decode of a host batch (uint8 bytes, int64 offsets[n+1]); asynchronous."""
         assert data.dtype == np.uint8 and offsets.dtype == np.int64
         self.n = len(offsets) - 1
+        self._submit_no += 1
         self._in_data, self._in_off = data, offsets
         self._check(self.lib.ck_submit(self.h, ptr(data), ptr(offsets), self.n))
 
     def submit_recordbatch(self, buf: np.ndarray) -> int:
         """H2D + CRC32C check + record split + field decode + walk of a fetch response's record set (concatenated Kafka
-        RecordBatch v2 frames, uncompressed); returns the number of records.  Column spans are relative to each VALUE."""
+        RecordBatch v2 frames, uncompressed or compressed with gzip / LZ4, which are decompressed on the device); returns
+        the number of records.  Column spans are relative to each VALUE.  Raises EngineError if the submitted plus the
+        decompressed bytes exceed max_in_bytes."""
         assert buf.dtype == np.uint8
         n = C.c_uint32(0)
+        self._submit_no += 1
         self._check(self.lib.ck_submit_recordbatch(self.h, ptr(buf), buf.nbytes, C.byref(n)))
         self.n = n.value
         idx = self.rb_index()
-        # the host-side view of the batch for result decoding: record i = buf[val_off[i] : val_off[i] + val_len[i]]
-        self._in_data, self._in_off = buf, _SpanOffsets(idx["val_off"], idx["val_len"])
+        base, length = C.c_uint64(0), C.c_uint64(0)
+        self._check(self.lib.ck_fetch_rb_decompressed(self.h, None, 0, C.byref(base), C.byref(length)))
+        # the host-side view of the batch for result decoding: record i = data[val_off[i] : val_off[i] + val_len[i]]
+        data = _RecordBatchBytes(self, buf, base.value) if length.value else buf
+        self._in_data, self._in_off = data, _SpanOffsets(idx["val_off"], idx["val_len"])
         self._rb = idx
         return self.n
 
+    def rb_decompressed(self) -> np.ndarray:
+        """the decompressed records sections of the last submit_recordbatch (one device-to-host copy); they start at
+        offset `len(buf)` rounded up to 16 of the space rb_index() offsets index.  Empty if no frame was compressed."""
+        base, length = C.c_uint64(0), C.c_uint64(0)
+        self._check(self.lib.ck_fetch_rb_decompressed(self.h, None, 0, C.byref(base), C.byref(length)))
+        out = np.empty(max(length.value, 1), dtype=np.uint8)
+        if length.value:
+            self._check(self.lib.ck_fetch_rb_decompressed(self.h, ptr(out), out.nbytes, C.byref(base), C.byref(length)))
+        return out[:length.value]
+
+    def rb_bytes(self) -> np.ndarray | _RecordBatchBytes:
+        """the byte space rb_index() offsets index (slice it as data[start:stop]): the submitted buffer, followed by the
+        decompressed records sections of its compressed frames"""
+        return self._in_data
+
     def rb_index(self) -> dict[str, np.ndarray]:
-        """where value / key / the correlation_id header of every record lie in the submitted buffer (len -1 = absent)"""
+        """where value / key / the correlation_id header of every record lie (len -1 = absent): offsets into the submitted
+        buffer followed by the decompressed sections of compressed frames (see rb_bytes()).  bad: 0, or why the record's
+        frame was refused — 1 CRC / framing / decompression failure, 2 a codec not decoded on the device (snappy, zstd)"""
         n = self.n
         out = {"val_off": np.zeros(n, np.int64), "val_len": np.zeros(n, np.uint32), "key_off": np.zeros(n, np.int64),
                "key_len": np.zeros(n, np.int32), "corr_off": np.zeros(n, np.int64), "corr_len": np.zeros(n, np.int32),
@@ -326,6 +377,7 @@ class BatchEngine:
                       host_off: np.ndarray | None = None) -> None:
         """decode a batch already resident in HBM (torch tensors or raw device addresses)."""
         self.n = n
+        self._submit_no += 1
         self._in_data, self._in_off = host_data, host_off
         a = dev_data if isinstance(dev_data, int) else ptr(dev_data)
         b = dev_off if isinstance(dev_off, int) else ptr(dev_off)

@@ -47,6 +47,8 @@ struct ck_handle {
     long long *d_rb_batch_off = nullptr, *d_rb_rec_pos = nullptr, *d_rb_key_off = nullptr, *d_rb_corr_off = nullptr, *d_rb_rec_off = nullptr, *d_rb_frame_len = nullptr;
     u32 *d_rb_rec_base = nullptr, *d_rb_batch_bad = nullptr, *d_rb_rec_batch = nullptr, *d_rb_val_len = nullptr, *d_rb_rec_bad = nullptr, *d_rb_idx = nullptr, *d_rb_sizes = nullptr, *d_rb_partial = nullptr;
     int *d_rb_key_len = nullptr, *d_rb_corr_len = nullptr; u8* d_rb_frame = nullptr; uint64_t rb_frame_cap = 0; uint32_t rb_n = 0;
+    long long *d_rb_slot = nullptr, *d_rb_sec_off = nullptr; u32 *d_rb_dlen = nullptr, *d_rb_sec_len = nullptr;   // compressed batches
+    uint64_t rb_dbase = 0, rb_dlen = 0;      // decompressed sections of the last fetch: d_in[rb_dbase .. + rb_dlen)
     // exchange planning (allocated on first use)
     u32* d_x_hist = nullptr; long long* d_x_base = nullptr; unsigned long long* d_x_nbytes = nullptr;
     long long *d_x_src_off = nullptr, *d_x_len = nullptr, *d_x_dst_off = nullptr; u32 *d_x_len32 = nullptr, *d_x_pub = nullptr;
@@ -176,7 +178,8 @@ extern "C" void ck_destroy(ck_handle* h) {
     void* gptrs[] = {h->gate.keys, h->gate.vals, h->gate.entries, h->gate.slots, h->gate.arena, h->gate.ctr, h->d_rec_entry,
                      h->d_rb_batch_off, h->d_rb_rec_pos, h->d_rb_key_off, h->d_rb_corr_off, h->d_rb_rec_off, h->d_rb_frame_len, h->d_rb_rec_base, h->d_rb_batch_bad,
                      h->d_g_hist, h->d_g_o1, h->d_g_o2, h->d_g_keys, h->d_g_base, h->d_g_tile, h->d_g_grand,
-                     h->d_rb_rec_batch, h->d_rb_val_len, h->d_rb_rec_bad, h->d_rb_idx, h->d_rb_sizes, h->d_rb_partial, h->d_rb_key_len, h->d_rb_corr_len, h->d_rb_frame};
+                     h->d_rb_rec_batch, h->d_rb_val_len, h->d_rb_rec_bad, h->d_rb_idx, h->d_rb_sizes, h->d_rb_partial, h->d_rb_key_len, h->d_rb_corr_len, h->d_rb_frame,
+                     h->d_rb_slot, h->d_rb_sec_off, h->d_rb_dlen, h->d_rb_sec_len};
     for (void* p : gptrs) if (p) cudaFree(p);
     for (u32 d = 0; d < CK_X_MAXWORLD; d++) if (h->peer_opened[d]) cudaIpcCloseMemHandle(h->peer_opened[d]);
     if (h->d_recv) cudaFree(h->d_recv);
@@ -659,47 +662,119 @@ static int rb_alloc(ck_handle* h) {
     CUDA_TRY(h, cudaMalloc((void**)&h->d_rb_rec_bad, sizeof(u32) * mr));
     return 0;
 }
+static int rb_alloc_codec(ck_handle* h) {
+    if (h->d_rb_slot) return 0;
+    size_t mr = (size_t)h->max_records + 1;
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rb_slot, sizeof(long long) * (mr + 1)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rb_sec_off, sizeof(long long) * mr));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rb_dlen, sizeof(u32) * mr));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rb_sec_len, sizeof(u32) * mr));
+    return 0;
+}
 static inline uint32_t host_be32(const uint8_t* p) { return ((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | p[3]; }
 
 // A fetch response's record set (concatenated RecordBatch v2 frames, as it came off the socket) goes to HBM in one copy;
 // CRC32C check, record split and varint field decode run on the device and the walker reads every value where it lies.
 // The host only chains through the frame headers (12 + batchLength bytes each) to index the frames.
+// Frames compressed with gzip (codec 1) or LZ4 (codec 3) are decompressed on the device into 16-byte aligned slots of
+// the input buffer right after the submitted bytes; their records are read there.  Such a fetch costs one more host
+// synchronisation (the decompressed total, to check it against max_in_bytes); a fetch without them takes the same path
+// as before.  Other codecs (snappy, zstd) leave their frames bad with reason CK_RB_BAD_CODEC.
 extern "C" int ck_submit_recordbatch(ck_handle* h, const uint8_t* host_buf, uint64_t nbytes, uint32_t* n_records) {
     cudaSetDevice(h->device);
     if (nbytes > h->max_in) return fail(h, "ck_submit_recordbatch: buffer larger than max_in_bytes");
     if (rb_alloc(h)) return 1;
     std::vector<long long> boff; std::vector<u32> rbase;
     uint64_t pos = 0; uint64_t total = 0;
+    bool compressed = false;
     while (pos + 12 <= nbytes) {
         uint32_t blen = host_be32(host_buf + pos + 8);
         uint64_t end = pos + 12 + (uint64_t)blen;
         if ((int32_t)blen < (int32_t)(CK_RB_HEADER - 12) || end > nbytes) break;         // truncated trailing frame: legal in a fetch response
         uint32_t cnt = host_be32(host_buf + pos + 57);
         if (total + cnt > h->max_records) return fail(h, "ck_submit_recordbatch: more records than max_records");
+        uint32_t codec = host_buf[pos + 22] & 7u;
+        compressed |= codec == CK_RB_GZIP || codec == CK_RB_LZ4;
         boff.push_back((long long)pos); rbase.push_back((u32)total);
         total += cnt; pos = end;
     }
     boff.push_back((long long)pos); rbase.push_back((u32)total);
     u32 nb = (u32)boff.size() - 1, n = (u32)total;
     if (n_records) *n_records = n;
+    if (compressed && rb_alloc_codec(h)) return 1;
+    h->rb_dbase = 0; h->rb_dlen = 0;
     CUDA_TRY(h, cudaMemcpyAsync(h->d_in, host_buf, pos, cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaMemsetAsync(h->d_in + pos, 0, 16, h->stream));
     CUDA_TRY(h, cudaMemcpyAsync(h->d_rb_batch_off, boff.data(), sizeof(long long) * (nb + 1), cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaMemcpyAsync(h->d_rb_rec_base, rbase.data(), sizeof(u32) * (nb + 1), cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));           // the two index vectors are pageable stack objects
     h->rb_n = n;
-    if (nb) {
+    if (nb && !compressed) {
         KTimer t(h, CK_K_WALK);
         CKL(h) ck_rb_crc_kernel<<<(nb + 7) / 8, 256, 0, h->stream>>>(h->d_in, h->d_rb_batch_off, nb, h->d_rb_batch_bad);
-        CKL(h) ck_rb_split_kernel<<<(nb + 127) / 128, 128, 0, h->stream>>>(h->d_in, h->d_rb_batch_off, h->d_rb_rec_base, nb, h->d_rb_batch_bad,
-                                                                        h->d_rb_rec_pos, h->d_rb_rec_batch);
+        CKL(h) ck_rb_split_kernel<<<(nb + 127) / 128, 128, 0, h->stream>>>(h->d_in, h->d_rb_batch_off, h->d_rb_rec_base, nb, nullptr, nullptr,
+                                                                        h->d_rb_batch_bad, h->d_rb_rec_pos, h->d_rb_rec_batch);
         if (n) CKL(h) ck_rb_fields_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->d_in, (long long)pos, h->d_rb_rec_pos, h->d_rb_rec_batch, h->d_rb_batch_bad, n,
             h->d_in_off, h->d_rb_val_len, h->d_rb_key_off, h->d_rb_key_len, h->d_rb_corr_off, h->d_rb_corr_len, h->d_rb_rec_bad);
         CUDA_TRY(h, cudaGetLastError());
+    } else if (nb) {
+        // CRC, size pass, scan of the slot sizes, capacity check (the one extra synchronisation), decompress, split
+        {
+            KTimer t(h, CK_K_WALK);
+            CKL(h) ck_rb_crc_kernel<<<(nb + 7) / 8, 256, 0, h->stream>>>(h->d_in, h->d_rb_batch_off, nb, h->d_rb_batch_bad);
+            CUDA_TRY(h, cudaGetLastError());
+        }
+        {
+            KTimer t(h, CK_K_CODEC);
+            CKL(h) ck_rb_csize_kernel<<<(nb + 127) / 128, 128, 0, h->stream>>>(h->d_in, h->d_rb_batch_off, nb, h->d_rb_batch_bad, h->d_rb_dlen);
+            CUDA_TRY(h, cudaGetLastError());
+        }
+        if (run_scan(h, h->d_rb_dlen, nb, h->d_rb_slot, 15)) return 1;
+        unsigned long long dtotal = 0;
+        CUDA_TRY(h, cudaMemcpyAsync(h->h_grand, h->d_grand, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+        dtotal = *h->h_grand;
+        uint64_t dbase = (pos + 15) & ~15ull;
+        if (dbase + dtotal > h->max_in) {
+            char b[256];
+            snprintf(b, sizeof b, "ck_submit_recordbatch: %llu submitted + %llu decompressed bytes (with padding) exceed max_in_bytes = %llu",
+                     (unsigned long long)pos, dtotal, (unsigned long long)h->max_in);
+            h->rb_n = 0; h->n = 0;
+            return fail(h, b);
+        }
+        {
+            KTimer t(h, CK_K_CODEC);
+            CKL(h) ck_rb_decompress_kernel<<<(nb + 127) / 128, 128, 0, h->stream>>>(h->d_in, h->d_rb_batch_off, nb, (long long)dbase, h->d_rb_slot,
+                                                                                 h->d_rb_dlen, h->d_rb_batch_bad, h->d_rb_sec_off, h->d_rb_sec_len);
+            CUDA_TRY(h, cudaGetLastError());
+        }
+        CUDA_TRY(h, cudaMemsetAsync(h->d_in + dbase + dtotal, 0, 16, h->stream));
+        h->rb_dbase = dbase; h->rb_dlen = dtotal;
+        {
+            KTimer t(h, CK_K_WALK);
+            CKL(h) ck_rb_split_kernel<<<(nb + 127) / 128, 128, 0, h->stream>>>(h->d_in, h->d_rb_batch_off, h->d_rb_rec_base, nb, h->d_rb_sec_off,
+                                                                            h->d_rb_sec_len, h->d_rb_batch_bad, h->d_rb_rec_pos, h->d_rb_rec_batch);
+            if (n) CKL(h) ck_rb_fields_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(h->d_in, (long long)(dbase + dtotal), h->d_rb_rec_pos, h->d_rb_rec_batch,
+                h->d_rb_batch_bad, n, h->d_in_off, h->d_rb_val_len, h->d_rb_key_off, h->d_rb_key_len, h->d_rb_corr_off, h->d_rb_corr_len, h->d_rb_rec_bad);
+            CUDA_TRY(h, cudaGetLastError());
+        }
     }
     h->cur_in = h->d_in; h->cur_in_off = h->d_in_off; h->cur_len = h->d_rb_val_len; h->n = n; h->n_payloads = 0; h->n_pubs = 0;
     if (launch_decode(h)) return 1;
     if (n) { CKL(h) ck_rb_mark_bad_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(h->d_rb_rec_bad, n, h->d_cols, n); CUDA_TRY(h, cudaGetLastError()); }
+    return 0;
+}
+
+// the decompressed records sections of the last ck_submit_recordbatch: host_dst[0 .. *len) = input bytes [*base, *base + *len)
+// (the offsets ck_fetch_rb_index reports for records of compressed frames lie there); *len = 0 when no frame was compressed
+extern "C" int ck_fetch_rb_decompressed(ck_handle* h, uint8_t* host_dst, uint64_t cap, uint64_t* base, uint64_t* len) {
+    cudaSetDevice(h->device);
+    if (base) *base = h->rb_dbase;
+    if (len) *len = h->rb_dlen;
+    if (!h->rb_dlen || !host_dst) return 0;
+    if (h->rb_dlen > cap) return fail(h, "ck_fetch_rb_decompressed: host buffer too small");
+    CUDA_TRY(h, cudaMemcpyAsync(host_dst, h->d_in + h->rb_dbase, h->rb_dlen, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     return 0;
 }
 

@@ -11,6 +11,9 @@
 //   ck_rb_split_kernel   thread per batch: hop from record to record (each starts with its own varint length)
 //   ck_rb_fields_kernel  thread per record: zig-zag varints -> key span, value span, the `correlation_id` header span
 // The walker then reads every value where it lies inside the raw buffer (ck_view.len): no per-record slicing on the host.
+// Compressed frames (gzip = codec 1, ck_inflate.cuh; LZ4 = codec 3, ck_lz4.cuh), only when a fetch holds any:
+//   ck_rb_csize_kernel       thread per frame: decompressed size (gzip ISIZE / LZ4 token walk); scan -> 16-byte slots
+//   ck_rb_decompress_kernel  thread per frame: decode into the slot after the submitted bytes; the split then reads there
 //
 // encode (produce): the payloads of one topic-partition (an index list the producer side already has) become one frame:
 //   ck_rb_size_kernel    thread per record: encoded size (varints depend on the record's offsetDelta = its rank)
@@ -20,40 +23,62 @@
 #ifndef CK_KAFKA_CUH
 #define CK_KAFKA_CUH
 
-#define CK_CRC_POLY 0x82F63B78u
+#include "ck_walk.cuh"            // u8 / u32 and CK_HD (the CRC and checksum cores below also build on the host)
+
+#define CK_CRC_POLY 0x82F63B78u      // CRC32C (Castagnoli), reflected: the RecordBatch CRC
+#define CK_CRC32_POLY 0xEDB88320u    // CRC-32 (IEEE 802.3), reflected: the gzip trailer (ck_inflate.cuh)
 #define CK_RB_HEADER 61u
 #define CK_RB_CRC_FROM 21u
 
-// ---- CRC32C -----------------------------------------------------------------------------------------------------------
-// four 256-entry tables (slicing-by-4) built in shared memory by the block itself
-__device__ __forceinline__ void ck_crc_tables(u32* t /* [4][256] */) {
-    for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
+// ---- CRC32C / CRC-32 -------------------------------------------------------------------------------------------------
+// four 256-entry tables (slicing-by-4) for the reflected polynomial `poly`, built in shared memory by the block itself
+// (by the calling thread alone in the host test build)
+CK_HD void ck_crc_tables(u32* t /* [4][256] */, u32 poly = CK_CRC_POLY) {
+#if defined(__CUDA_ARCH__)
+    const u32 i0 = threadIdx.x, step = blockDim.x;
+#else
+    const u32 i0 = 0, step = 1;
+#endif
+    for (u32 i = i0; i < 256; i += step) {
         u32 c = i;
 #pragma unroll
-        for (int k = 0; k < 8; k++) c = (c >> 1) ^ ((c & 1u) ? CK_CRC_POLY : 0u);
+        for (int k = 0; k < 8; k++) c = (c >> 1) ^ ((c & 1u) ? poly : 0u);
         t[i] = c;
     }
+#if defined(__CUDA_ARCH__)
     __syncthreads();
-    for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
+#endif
+    for (u32 i = i0; i < 256; i += step) {
         u32 c = t[i];
 #pragma unroll
         for (int k = 1; k < 4; k++) { c = (c >> 8) ^ t[c & 0xffu]; t[k * 256 + i] = c; }
     }
+#if defined(__CUDA_ARCH__)
     __syncthreads();
+#endif
 }
-// finalised CRC32C of p[0..n) (init / xor-out all ones)
-__device__ __forceinline__ u32 ck_crc32c_span(const u32* __restrict__ t, const u8* __restrict__ p, u32 n) {
+// finalised CRC of p[0..n) (init / xor-out all ones) for the polynomial the tables were built for
+CK_HD u32 ck_crc_span(const u32* __restrict__ t, const u8* __restrict__ p, u32 n) {
     u32 c = 0xffffffffu;
     while (n && ((uintptr_t)p & 3u)) { c = t[(c ^ *p++) & 0xffu] ^ (c >> 8); n--; }
     const u32* w = (const u32*)p;
     for (; n >= 4; n -= 4) {
+#if defined(__CUDA_ARCH__)
         c ^= __ldg(w++);
+#else
+        c ^= *w++;
+#endif
         c = t[768 + (c & 0xffu)] ^ t[512 + ((c >> 8) & 0xffu)] ^ t[256 + ((c >> 16) & 0xffu)] ^ t[c >> 24];
     }
     p = (const u8*)w;
     while (n--) c = t[(c ^ *p++) & 0xffu] ^ (c >> 8);
     return ~c;
 }
+
+#include "ck_inflate.cuh"
+#include "ck_lz4.cuh"
+
+#if defined(__CUDACC__)
 // a(x) * b(x) mod P(x), reflected representation (bit 31 = x^0)
 __device__ __forceinline__ u32 ck_gf_mul(u32 a, u32 b) {
     u32 p = 0;
@@ -78,7 +103,7 @@ __device__ __forceinline__ u32 ck_crc_combine(u32 crc_a, u32 crc_b, u32 xpow_len
 __device__ __forceinline__ u32 ck_crc32c_warp(const u32* __restrict__ t, const u8* __restrict__ p, u32 n, u32 lane) {
     u32 chunk = (n >> 5) & ~3u;
     u32 head = n - 31u * chunk;
-    u32 c = lane == 0 ? ck_crc32c_span(t, p, head) : (chunk ? ck_crc32c_span(t, p + head + (lane - 1) * chunk, chunk) : 0u);
+    u32 c = lane == 0 ? ck_crc_span(t, p, head) : (chunk ? ck_crc_span(t, p + head + (lane - 1) * chunk, chunk) : 0u);
     if (!chunk) return __shfl_sync(0xffffffffu, c, 0);
     u32 xp = ck_gf_xpow8(chunk);               // x^(8 chunk); squared at every level: right blocks hold 1, 2, 4, 8, 16 chunks
 #pragma unroll
@@ -95,6 +120,13 @@ __device__ __forceinline__ void ck_put_be32(u8* p, u32 v) { p[0] = v >> 24; p[1]
 __device__ __forceinline__ void ck_put_be64(u8* p, unsigned long long v) { ck_put_be32(p, (u32)(v >> 32)); ck_put_be32(p + 4, (u32)v); }
 
 // ---- decode -------------------------------------------------------------------------------------------------------------
+// batch_bad[b] / rec_bad[i]: why a frame (and every record in it) was refused
+#define CK_RB_BAD 1u          // CRC32C, framing or decompression failure
+#define CK_RB_BAD_CODEC 2u    // a compression codec the device does not decode (snappy = 2, zstd = 4, 5-7 unassigned)
+#define CK_RB_GZIP 1u
+#define CK_RB_LZ4 3u
+__device__ __forceinline__ bool ck_rb_codec_decoded(u32 codec) { return codec == 0 || codec == CK_RB_GZIP || codec == CK_RB_LZ4; }
+
 // batch_off[b] .. batch_off[b+1]: frame b inside buf (indexed by the host: the frames chain through their own length field)
 __global__ void __launch_bounds__(256)
 ck_rb_crc_kernel(const u8* __restrict__ buf, const long long* __restrict__ batch_off, u32 nb, u32* __restrict__ batch_bad) {
@@ -105,10 +137,11 @@ ck_rb_crc_kernel(const u8* __restrict__ buf, const long long* __restrict__ batch
     const u8* f = buf + batch_off[w];
     u32 flen = (u32)(batch_off[w + 1] - batch_off[w]);
     u32 bad = 0;
-    if (flen < CK_RB_HEADER || f[16] != 2 || ((f[21] << 8 | f[22]) & 7)) bad = 1;      // not magic 2 / compressed: not handled here
+    if (flen < CK_RB_HEADER || f[16] != 2) bad = CK_RB_BAD;                            // not magic 2
     else {
         u32 c = ck_crc32c_warp(t, f + CK_RB_CRC_FROM, flen - CK_RB_CRC_FROM, lane);
-        if (c != ck_be32(f + 17)) bad = 1;
+        if (c != ck_be32(f + 17)) bad = CK_RB_BAD;
+        else if (!ck_rb_codec_decoded(f[22] & 7u)) bad = CK_RB_BAD_CODEC;
     }
     if (lane == 0) batch_bad[w] = bad;
 }
@@ -127,28 +160,73 @@ __device__ __forceinline__ bool ck_varint(const u8* __restrict__ p, u32& pos, u3
 }
 
 // thread per batch: where does each record start.  rec_base[b] = records in the batches before b (host prefix sum of
-// the recordsCount header fields); a batch whose records do not add up to its length is marked bad
+// the recordsCount header fields).  The records of batch b are the section sec_off[b] .. + sec_len[b] of buf: the raw
+// bytes after the header, or for a compressed batch its decompressed slot; sec_off = nullptr means every batch is
+// uncompressed (the section is the rest of the frame).  A batch whose records do not exactly fill its section is bad.
 __global__ void __launch_bounds__(128)
 ck_rb_split_kernel(const u8* __restrict__ buf, const long long* __restrict__ batch_off, const u32* __restrict__ rec_base, u32 nb,
+                   const long long* __restrict__ sec_off, const u32* __restrict__ sec_len,
                    u32* __restrict__ batch_bad, long long* __restrict__ rec_pos, u32* __restrict__ rec_batch) {
     u32 b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= nb) return;
     u32 r0 = rec_base[b], cnt = rec_base[b + 1] - r0;
-    long long base = batch_off[b];
+    long long base = sec_off ? sec_off[b] : batch_off[b] + CK_RB_HEADER;
+    u32 slen = sec_off ? sec_len[b] : (u32)(batch_off[b + 1] - batch_off[b]) - CK_RB_HEADER;
     const u8* f = buf + base;
-    u32 flen = (u32)(batch_off[b + 1] - base);
-    u32 pos = CK_RB_HEADER;
+    u32 pos = 0;
     bool ok = !batch_bad[b];
     for (u32 k = 0; k < cnt; k++) {
         rec_batch[r0 + k] = b;
         if (!ok) { rec_pos[r0 + k] = -1; continue; }
         rec_pos[r0 + k] = base + pos;
         long long len;
-        if (!ck_varint(f, pos, flen, len) || len < 0 || pos + (u32)len > flen) { ok = false; rec_pos[r0 + k] = -1; continue; }
+        if (!ck_varint(f, pos, slen, len) || len < 0 || pos + (u32)len > slen) { ok = false; rec_pos[r0 + k] = -1; continue; }
         pos += (u32)len;
     }
-    if (ok && pos != flen) ok = false;
-    if (!ok) batch_bad[b] = 1;
+    if (ok && pos != slen) ok = false;
+    if (!ok && !batch_bad[b]) batch_bad[b] = CK_RB_BAD;
+}
+
+// thread per batch, compressed fetches only (after the CRC kernel): the decompressed size of every compressed batch that
+// passed its CRC — gzip: the trailer's ISIZE (checked after the inflate); LZ4: a walk over the block headers and tokens,
+// cross-checked against a stored content size.  dlen[b] = 0 for the others; a batch whose size cannot be had is bad.
+__global__ void __launch_bounds__(128)
+ck_rb_csize_kernel(const u8* __restrict__ buf, const long long* __restrict__ batch_off, u32 nb, u32* __restrict__ batch_bad,
+                   u32* __restrict__ dlen) {
+    u32 b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nb) return;
+    const u8* f = buf + batch_off[b];
+    u32 codec = f[22] & 7u, n = 0;
+    if (!batch_bad[b] && codec) {
+        const u8* src = f + CK_RB_HEADER;
+        u32 slen = (u32)(batch_off[b + 1] - batch_off[b]) - CK_RB_HEADER;
+        bool ok = codec == CK_RB_GZIP ? ck_gzip_isize(src, slen, n) : ck_lz4_frame<false>(src, slen, nullptr, n);
+        if (!ok || n > 0x7fff0000u) { batch_bad[b] = CK_RB_BAD; n = 0; }
+    }
+    dlen[b] = n;
+}
+
+// thread per batch: decompress every compressed batch into its slot dbase + slot[b] (exclusive scan of dlen rounded up
+// to 16) and give every batch its records section for the split.  A batch that does not decode is bad.
+__global__ void __launch_bounds__(128)
+ck_rb_decompress_kernel(u8* __restrict__ buf, const long long* __restrict__ batch_off, u32 nb, long long dbase,
+                        const long long* __restrict__ slot, const u32* __restrict__ dlen, u32* __restrict__ batch_bad,
+                        long long* __restrict__ sec_off, u32* __restrict__ sec_len) {
+    __shared__ u32 t[1024];
+    ck_crc_tables(t, CK_CRC32_POLY);
+    u32 b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nb) return;
+    long long fo = batch_off[b];
+    const u8* f = buf + fo;
+    u32 flen = (u32)(batch_off[b + 1] - fo);
+    u32 codec = flen >= CK_RB_HEADER ? f[22] & 7u : 0u;
+    if (!codec || batch_bad[b]) { sec_off[b] = fo + CK_RB_HEADER; sec_len[b] = flen >= CK_RB_HEADER ? flen - CK_RB_HEADER : 0u; return; }
+    u32 n = dlen[b];
+    u8* dst = buf + dbase + slot[b];
+    const u8* src = f + CK_RB_HEADER;
+    bool ok = codec == CK_RB_GZIP ? ck_gunzip(src, flen - CK_RB_HEADER, dst, n, t) : ck_lz4_frame<true>(src, flen - CK_RB_HEADER, dst, n);
+    if (!ok) batch_bad[b] = CK_RB_BAD;
+    sec_off[b] = dbase + slot[b]; sec_len[b] = n;
 }
 
 // thread per record
@@ -161,7 +239,7 @@ ck_rb_fields_kernel(const u8* __restrict__ buf, long long buf_len, const long lo
     if (i >= n) return;
     val_off[i] = 0; val_len[i] = 0; key_off[i] = 0; key_len[i] = -1; corr_off[i] = 0; corr_len[i] = -1;
     long long rp = rec_pos[i];
-    if (rp < 0 || batch_bad[rec_batch[i]]) { rec_bad[i] = 1; return; }
+    if (rp < 0 || batch_bad[rec_batch[i]]) { u32 why = batch_bad[rec_batch[i]]; rec_bad[i] = why ? why : CK_RB_BAD; return; }
     const u8* p = buf + rp;
     u32 end = (u32)min((long long)0x7fffffff, buf_len - rp), pos = 0;
     long long len, t;
@@ -323,4 +401,5 @@ __global__ void ck_rb_crc_fold_kernel(u8* __restrict__ frame, const long long* _
     ck_put_be32(frame + 17, c);
 }
 
+#endif  // __CUDACC__
 #endif  // CK_KAFKA_CUH

@@ -84,16 +84,22 @@ int  ck_fetch_groups(ck_handle* h, uint32_t* host_order, uint32_t* host_key_coun
 
 /* Kafka RecordBatch v2 framing on the device (reference: aiokafka under broker.subscriber / broker.publish,
  * calfkit/worker/worker.py:45-53, calfkit/nodes/base.py:82-87).  ck_submit_recordbatch takes a fetch response's record set
- * (concatenated v2 frames, uncompressed) as it came off the socket: one H2D copy, then CRC32C verification, record split and
- * zig-zag varint field decode on the device; the walker reads each value where it lies.  Records of a frame that fails the
- * CRC / framing check get status 6 (bad frame); a truncated trailing frame is ignored.  *n_records = records decoded.
- * ck_fetch_rb_index: per record, where value / key / the `correlation_id` header lie in the submitted buffer (-1 = absent).
+ * (concatenated v2 frames) as it came off the socket: one H2D copy, then CRC32C verification, record split and zig-zag
+ * varint field decode on the device; the walker reads each value where it lies.  Frames compressed with gzip (codec 1) or
+ * LZ4 (codec 3) are decompressed on the device into 16-byte aligned slots of the input buffer right after the submitted
+ * bytes (one extra host synchronisation, paid only by fetches that hold such frames; submitted + decompressed bytes must fit
+ * max_in_bytes).  Records of a frame that fails the CRC / framing / decompression check, or whose codec is not decoded on
+ * the device (snappy, zstd), get status 6 (bad frame); a truncated trailing frame is ignored.  *n_records = records decoded.
+ * ck_fetch_rb_index: per record, where value / key / the `correlation_id` header lie (-1 = absent), as offsets into the
+ * submitted buffer followed by the decompressed sections; bad = 0, 1 (CRC / framing / decompression) or 2 (codec).
+ * ck_fetch_rb_decompressed: host_dst[0 .. *len) = the decompressed sections, which start at offset *base of that space.
  * ck_encode_recordbatch: the publishes host_idx[0..n) of the current plan (one topic-partition, in send order) -> one
  * uncompressed v2 frame (offsetDelta = position in the list, key = correlation id when keyed, headers content-type and
  * correlation_id, CRC32C), built on the device and copied to host_frame. */
 int  ck_submit_recordbatch(ck_handle* h, const uint8_t* host_buf, uint64_t nbytes, uint32_t* n_records);
 int  ck_fetch_rb_index(ck_handle* h, int64_t* val_off, uint32_t* val_len, int64_t* key_off, int32_t* key_len,
                        int64_t* corr_off, int32_t* corr_len, uint32_t* bad);
+int  ck_fetch_rb_decompressed(ck_handle* h, uint8_t* host_dst, uint64_t cap, uint64_t* base, uint64_t* len);
 int  ck_encode_recordbatch(ck_handle* h, const uint32_t* host_idx, uint32_t n, int64_t base_offset, int64_t timestamp_ms,
                            uint8_t* host_frame, uint64_t cap, uint64_t* frame_len);
 
@@ -221,7 +227,7 @@ int  ck_device_buffers2(ck_handle* h, void** pubs, void** pay_len, void** descs)
 int  ck_profile(ck_handle* h, int enable);         /* record (asynchronous) CUDA events around every kernel */
 int  ck_profile_read(ck_handle* h, float* ms /* CK_NUM_KERNELS */, uint32_t* launches /* CK_NUM_KERNELS */, int reset);
 
-enum { CK_K_WALK = 0, CK_K_PLAN, CK_K_SCAN, CK_K_EMIT, CK_K_ROUTE, CK_K_FANOUT, CK_K_CANON, CK_K_WALK_LONG, CK_K_WALK_ELEMS, CK_NUM_KERNELS };
+enum { CK_K_WALK = 0, CK_K_PLAN, CK_K_SCAN, CK_K_EMIT, CK_K_ROUTE, CK_K_FANOUT, CK_K_CANON, CK_K_WALK_LONG, CK_K_WALK_ELEMS, CK_K_CODEC, CK_NUM_KERNELS };
 
 #ifdef __cplusplus
 }
