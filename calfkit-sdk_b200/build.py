@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "libcalfkit_b200.so")
 SRCS = [os.path.join(HERE, "csrc", "ck_api.cu")]
-DEPS = SRCS + [os.path.join(HERE, "csrc", f) for f in ("ck_kernels.cuh", "ck_walk.cuh", "ck_float.cuh", "ck_canon.cuh", "ck_plan2.cuh", "ck_gate.cuh", "ck_kafka.cuh", "ck_inflate.cuh", "ck_lz4.cuh", "ck_group.cuh", "ck_xsend.cuh", "ck_fanout2.cuh", "ck_walk_long.cuh", "ck_common.h")] + \
+DEPS = SRCS + [os.path.join(HERE, "csrc", f) for f in ("ck_kernels.cuh", "ck_walk.cuh", "ck_float.cuh", "ck_canon.cuh", "ck_plan2.cuh", "ck_gate.cuh", "ck_kafka.cuh", "ck_inflate.cuh", "ck_lz4.cuh", "ck_lz4_enc.cuh", "ck_deflate.cuh", "ck_group.cuh", "ck_xsend.cuh", "ck_fanout2.cuh", "ck_walk_long.cuh", "ck_common.h")] + \
     [os.path.join(HERE, "..", "include", "calfkit_b200.h")]
 
 

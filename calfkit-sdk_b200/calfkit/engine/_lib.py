@@ -42,7 +42,7 @@ EXPORTS = ["ck_create", "ck_destroy", "ck_last_error", "ck_version", "ck_registe
            "ck_device_buffers", "ck_device_buffers2", "ck_gather_spans", "ck_profile", "ck_profile_read", "ck_fetch_cols",
            "ck_host_alloc", "ck_host_free", "ck_canon_stats", "ck_fetch_output_async",
            "ck_fetch_cols_async", "ck_gate_create", "ck_gate_register", "ck_gate_arrive", "ck_gate_stats", "ck_gate_reset", "ck_submit_recordbatch",
-           "ck_fetch_rb_index", "ck_fetch_rb_decompressed", "ck_encode_recordbatch", "ck_group_publishes", "ck_fetch_groups", "ck_comm_create", "ck_comm_connect", "ck_exchange_send", "ck_recv_info", "ck_fetch_received", "ck_peek_received", "ck_fetch_received_async", "ck_set_option"]
+           "ck_fetch_rb_index", "ck_fetch_rb_decompressed", "ck_encode_recordbatch", "ck_encode_recordbatches", "ck_fetch_recordbatches", "ck_group_publishes", "ck_fetch_groups", "ck_comm_create", "ck_comm_connect", "ck_exchange_send", "ck_recv_info", "ck_fetch_received", "ck_peek_received", "ck_fetch_received_async", "ck_set_option"]
 
 _lib = None
 
@@ -104,6 +104,9 @@ def load() -> C.CDLL:
         "ck_fetch_rb_index": (C.c_int, [vp, i64p, u32p, i64p, i32p, i64p, i32p, u32p]),
         "ck_fetch_rb_decompressed": (C.c_int, [vp, u8p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "ck_encode_recordbatch": (C.c_int, [vp, u32p, C.c_uint32, C.c_int64, C.c_int64, u8p, C.c_uint64, C.POINTER(C.c_uint64)]),
+        "ck_encode_recordbatches": (C.c_int, [vp, u32p, C.c_uint32, u32p, C.c_uint32, i64p, C.c_int64, C.c_uint32, C.c_uint32,
+                                              C.POINTER(C.c_uint32), C.POINTER(C.c_uint64)]),
+        "ck_fetch_recordbatches": (C.c_int, [vp, u8p, C.c_uint64, vp, u32p]),
         "ck_gate_create": (C.c_int, [vp, C.c_uint32, C.c_uint32, C.c_uint64]),
         "ck_gate_register": (C.c_int, [vp, C.c_uint32]),
         "ck_gate_arrive": (C.c_int, [vp, C.c_uint64]),

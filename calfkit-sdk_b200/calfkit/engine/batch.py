@@ -373,6 +373,42 @@ class BatchEngine:
         self._check(self.lib.ck_encode_recordbatch(self.h, ptr(idx), len(idx), base_offset, timestamp_ms, ptr(buf), cap, C.byref(used)))
         return buf[:used.value]
 
+    _CODECS = {None: 0, "gzip": 1, "lz4": 3}
+
+    def encode_recordbatches(self, pub_indices: np.ndarray, group_sizes: Sequence[int] | None = None,
+                             base_offsets: Sequence[int] | None = None, timestamp_ms: int = 0,
+                             compression_type: str | None = None, max_batch_size: int = 16384
+                             ) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """the publishes `pub_indices` of the current plan, in groups of `group_sizes` consecutive indices (one
+        topic-partition each, in send order; None = one group), as runs of Kafka RecordBatch v2 frames built on the device:
+        a frame takes its group's next records while it stays within `max_batch_size` bytes (always at least one record),
+        and its records section is compressed with `compression_type` (None, "gzip" or "lz4", aiokafka's names).  Frame k
+        of group g starts at offset base_offsets[g] (default 0) plus the records of g in earlier frames.
+        Returns (data, frame_off, frame_group): frame i = data[frame_off[i]:frame_off[i + 1]], from group frame_group[i]."""
+        if compression_type not in self._CODECS:
+            raise ValueError(f"compression_type {compression_type!r} is not supported: use None, 'gzip' or 'lz4'")
+        if max_batch_size < 62:
+            raise ValueError(f"max_batch_size {max_batch_size} is below 62 (a 61-byte header and one record byte)")
+        idx = np.ascontiguousarray(pub_indices, dtype=np.uint32)
+        sizes = np.asarray([len(idx)] if group_sizes is None else list(group_sizes), dtype=np.int64)
+        if (sizes < 0).any() or int(sizes.sum()) != len(idx):
+            raise ValueError(f"group_sizes must be non-negative and sum to len(pub_indices) = {len(idx)}")
+        goff = np.zeros(len(sizes) + 1, dtype=np.uint32)
+        np.cumsum(sizes, out=goff[1:])
+        base = None
+        if base_offsets is not None:
+            base = np.ascontiguousarray(base_offsets, dtype=np.int64)
+            if len(base) != len(sizes):
+                raise ValueError(f"base_offsets must have one entry per group ({len(sizes)})")
+        nf, total = C.c_uint32(0), C.c_uint64(0)
+        self._check(self.lib.ck_encode_recordbatches(self.h, ptr(idx), len(idx), ptr(goff), len(sizes), ptr(base), timestamp_ms,
+                                                     self._CODECS[compression_type], max_batch_size, C.byref(nf), C.byref(total)))
+        data = np.empty(max(total.value, 1), dtype=np.uint8)
+        frame_off = np.zeros(nf.value + 1, dtype=np.uint64)
+        frame_group = np.zeros(max(nf.value, 1), dtype=np.uint32)
+        self._check(self.lib.ck_fetch_recordbatches(self.h, ptr(data), data.nbytes, ptr(frame_off), ptr(frame_group)))
+        return data[:total.value], frame_off.astype(np.int64), frame_group[:nf.value]
+
     def submit_device(self, dev_data, dev_off, n: int, host_data: np.ndarray | None = None,
                       host_off: np.ndarray | None = None) -> None:
         """decode a batch already resident in HBM (torch tensors or raw device addresses)."""

@@ -49,6 +49,13 @@ struct ck_handle {
     int *d_rb_key_len = nullptr, *d_rb_corr_len = nullptr; u8* d_rb_frame = nullptr; uint64_t rb_frame_cap = 0; uint32_t rb_n = 0;
     long long *d_rb_slot = nullptr, *d_rb_sec_off = nullptr; u32 *d_rb_dlen = nullptr, *d_rb_sec_len = nullptr;   // compressed batches
     uint64_t rb_dbase = 0, rb_dlen = 0;      // decompressed sections of the last fetch: d_in[rb_dbase .. + rb_dlen)
+    // runs of frames on the produce side (ck_encode_recordbatches, allocated on first use)
+    u32 *d_rbs_idx = nullptr, *d_rbs_goff = nullptr, *d_rbs_delta = nullptr, *d_rbs_size = nullptr, *d_rbs_open = nullptr, *d_rbs_fid = nullptr;
+    u32 *d_rbs_ffirst = nullptr, *d_rbs_nch = nullptr, *d_rbs_csz = nullptr, *d_rbs_ccrc = nullptr, *d_rbs_fsize = nullptr, *d_rbs_fgroup = nullptr, *d_rbs_tabs = nullptr;
+    long long *d_rbs_base = nullptr, *d_rbs_recoff = nullptr, *d_rbs_openx = nullptr, *d_rbs_foff = nullptr, *d_rbs_cbase = nullptr, *d_rbs_coff = nullptr;
+    u8 *d_rbs_plain = nullptr, *d_rbs_slots = nullptr, *d_rbs_out = nullptr; ck_dfl_tables* d_rbs_dtabs = nullptr;
+    unsigned long long *d_rbs_tile = nullptr, *d_rbs_grand = nullptr, *h_rbs = nullptr;   // h_rbs: pinned
+    uint64_t rbs_plain_cap = 0, rbs_out_cap = 0, rbs_chunk_cap = 0, rbs_total = 0; uint32_t rbs_pool = 0, rbs_nf = 0;
     // exchange planning (allocated on first use)
     u32* d_x_hist = nullptr; long long* d_x_base = nullptr; unsigned long long* d_x_nbytes = nullptr;
     long long *d_x_src_off = nullptr, *d_x_len = nullptr, *d_x_dst_off = nullptr; u32 *d_x_len32 = nullptr, *d_x_pub = nullptr;
@@ -179,8 +186,13 @@ extern "C" void ck_destroy(ck_handle* h) {
                      h->d_rb_batch_off, h->d_rb_rec_pos, h->d_rb_key_off, h->d_rb_corr_off, h->d_rb_rec_off, h->d_rb_frame_len, h->d_rb_rec_base, h->d_rb_batch_bad,
                      h->d_g_hist, h->d_g_o1, h->d_g_o2, h->d_g_keys, h->d_g_base, h->d_g_tile, h->d_g_grand,
                      h->d_rb_rec_batch, h->d_rb_val_len, h->d_rb_rec_bad, h->d_rb_idx, h->d_rb_sizes, h->d_rb_partial, h->d_rb_key_len, h->d_rb_corr_len, h->d_rb_frame,
-                     h->d_rb_slot, h->d_rb_sec_off, h->d_rb_dlen, h->d_rb_sec_len};
+                     h->d_rb_slot, h->d_rb_sec_off, h->d_rb_dlen, h->d_rb_sec_len,
+                     h->d_rbs_idx, h->d_rbs_goff, h->d_rbs_delta, h->d_rbs_size, h->d_rbs_open, h->d_rbs_fid, h->d_rbs_ffirst, h->d_rbs_nch,
+                     h->d_rbs_csz, h->d_rbs_ccrc, h->d_rbs_fsize, h->d_rbs_fgroup, h->d_rbs_tabs, h->d_rbs_base, h->d_rbs_recoff, h->d_rbs_openx,
+                     h->d_rbs_foff, h->d_rbs_cbase, h->d_rbs_coff, h->d_rbs_plain, h->d_rbs_slots, h->d_rbs_out, h->d_rbs_dtabs, h->d_rbs_tile,
+                     h->d_rbs_grand};
     for (void* p : gptrs) if (p) cudaFree(p);
+    if (h->h_rbs) cudaFreeHost(h->h_rbs);
     for (u32 d = 0; d < CK_X_MAXWORLD; d++) if (h->peer_opened[d]) cudaIpcCloseMemHandle(h->peer_opened[d]);
     if (h->d_recv) cudaFree(h->d_recv);
     if (h->d_x_overflow) cudaFree(h->d_x_overflow);
@@ -838,6 +850,152 @@ extern "C" int ck_encode_recordbatch(ck_handle* h, const uint32_t* host_idx, uin
     CUDA_TRY(h, cudaMemcpyAsync(host_frame, h->d_rb_frame, total, cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (frame_len) *frame_len = total;
+    return 0;
+}
+
+// Runs of frames (ck_encode_recordbatches): scratch sized from max_out / max_payloads for every publish a plan can hold
+// (up to two per payload).  plain: the records
+// sections back to back; slots: one per 64 KB chunk, at its plaintext offset + 64 * chunk
+// index (a compressed chunk never exceeds its input by 64 bytes); out: the frames.  The compression pool is a fixed
+// number of threads (128 per SM), each with a hash table and DEFLATE scratch of its own.
+static int rbs_alloc(ck_handle* h) {
+    if (h->d_rbs_idx) return 0;
+    size_t mp = (size_t)h->max_pubs + 1;
+    h->rbs_plain_cap = 2 * h->max_out + 256ull * h->max_pubs + 4096;
+    h->rbs_chunk_cap = h->rbs_plain_cap / CK_RBS_CHUNK + mp;
+    h->rbs_out_cap = h->rbs_plain_cap + 128ull * mp + 16ull * h->rbs_chunk_cap;
+    int sms = 0;
+    CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
+    h->rbs_pool = (u32)sms * 128u;
+    size_t big = mp > h->rbs_chunk_cap + 1 ? mp : h->rbs_chunk_cap + 1;
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_idx, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_goff, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_base, sizeof(long long) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_delta, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_size, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_open, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_fid, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_ffirst, sizeof(u32) * (mp + 1)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_nch, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_fsize, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_fgroup, sizeof(u32) * mp));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_recoff, sizeof(long long) * (mp + 1)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_openx, sizeof(long long) * (mp + 1)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_foff, sizeof(long long) * (mp + 1)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_cbase, sizeof(long long) * (mp + 1)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_csz, sizeof(u32) * h->rbs_chunk_cap));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_ccrc, sizeof(u32) * h->rbs_chunk_cap));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_coff, sizeof(long long) * (h->rbs_chunk_cap + 1)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_tile, sizeof(unsigned long long) * (big / CK_SCAN_TILE + 2)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_grand, sizeof(unsigned long long) * 4));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_plain, h->rbs_plain_cap + CK_PAD));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_slots, h->rbs_plain_cap + 64ull * h->rbs_chunk_cap + CK_PAD));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_out, h->rbs_out_cap + CK_PAD));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_tabs, sizeof(u32) * ((size_t)h->rbs_pool << CK_DFL_TAB_BITS)));
+    CUDA_TRY(h, cudaMalloc((void**)&h->d_rbs_dtabs, sizeof(ck_dfl_tables) * (size_t)h->rbs_pool));
+    CUDA_TRY(h, cudaMallocHost((void**)&h->h_rbs, sizeof(unsigned long long) * 4));
+    return 0;
+}
+
+// produce side, every (topic, partition) of a step in one call: groups of publishes -> runs of RecordBatch v2 frames split
+// to max_batch_bytes, records sections compressed with gzip or LZ4 on the device.  Two host synchronisations: after the
+// split (frame count, plaintext total) and, for compressed frames, after the scan of the compressed sizes.
+extern "C" int ck_encode_recordbatches(ck_handle* h, const uint32_t* host_idx, uint32_t n, const uint32_t* host_group_off,
+                                       uint32_t n_groups, const int64_t* host_base_offsets, int64_t timestamp_ms, uint32_t codec,
+                                       uint32_t max_batch_bytes, uint32_t* n_frames, uint64_t* total_bytes) {
+    cudaSetDevice(h->device);
+    h->rbs_nf = 0; h->rbs_total = 0;
+    if (codec != 0 && codec != CK_RB_GZIP && codec != CK_RB_LZ4) return fail(h, "ck_encode_recordbatches: codec must be 0 (none), 1 (gzip) or 3 (LZ4)");
+    if (max_batch_bytes < CK_RB_HEADER + 1) return fail(h, "ck_encode_recordbatches: max_batch_bytes must be at least 62");
+    if (n > h->max_pubs) return fail(h, "ck_encode_recordbatches: more indices than max_payloads * 2");
+    if (!n_groups || host_group_off[0] != 0 || host_group_off[n_groups] != n) return fail(h, "ck_encode_recordbatches: group offsets must run from 0 to n");
+    if (n_groups > h->max_pubs) return fail(h, "ck_encode_recordbatches: more groups than max_payloads * 2");
+    for (u32 g = 0; g < n_groups; g++) if (host_group_off[g + 1] < host_group_off[g]) return fail(h, "ck_encode_recordbatches: group offsets must not decrease");
+    for (u32 k = 0; k < n; k++) if (host_idx[k] >= h->n_pubs) return fail(h, "ck_encode_recordbatches: index outside the publish table");
+    if (rbs_alloc(h)) return 1;
+    if (!n) { if (n_frames) *n_frames = 0; if (total_bytes) *total_bytes = 0; return 0; }
+    CUDA_TRY(h, cudaMemcpyAsync(h->d_rbs_idx, host_idx, sizeof(u32) * n, cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->d_rbs_goff, host_group_off, sizeof(u32) * (n_groups + 1), cudaMemcpyHostToDevice, h->stream));
+    if (host_base_offsets) CUDA_TRY(h, cudaMemcpyAsync(h->d_rbs_base, host_base_offsets, sizeof(long long) * n_groups, cudaMemcpyHostToDevice, h->stream));
+    unsigned long long* gr = h->d_rbs_grand;                  // 0 plaintext bytes, 1 frames, 2 chunks, 3 output bytes
+    {
+        KTimer t(h, CK_K_EMIT);
+        CKL(h) ck_rbs_split_kernel<<<(n_groups + 7) / 8, 256, 0, h->stream>>>(h->d_pubs, h->d_rbs_idx, h->d_rbs_goff, n_groups, h->d_pay_len,
+                                                                            h->d_cols, h->n, max_batch_bytes, h->d_rbs_delta, h->d_rbs_size, h->d_rbs_open);
+        CUDA_TRY(h, cudaGetLastError());
+    }
+    if (run_scan(h, h->d_rbs_size, n, h->d_rbs_recoff, 0, h->d_rbs_tile, gr + 0)) return 1;
+    if (run_scan(h, h->d_rbs_open, n, h->d_rbs_openx, 0, h->d_rbs_tile, gr + 1)) return 1;
+    CUDA_TRY(h, cudaMemcpyAsync(h->h_rbs, gr, sizeof(unsigned long long) * 2, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    uint64_t plain = h->h_rbs[0]; u32 nf = (u32)h->h_rbs[1];
+    uint64_t cmax = plain / CK_RBS_CHUNK + nf;                // each frame adds at most one partial chunk
+    char msg[256];
+    if (plain > h->rbs_plain_cap || (!codec && plain + (uint64_t)CK_RB_HEADER * nf > h->rbs_out_cap) || cmax > h->rbs_chunk_cap) {
+        snprintf(msg, sizeof msg, "ck_encode_recordbatches: %llu bytes of records in %u frames exceed the scratch (%llu bytes of records, %llu bytes of frames)",
+                 (unsigned long long)plain, nf, (unsigned long long)h->rbs_plain_cap, (unsigned long long)h->rbs_out_cap);
+        return fail(h, msg);
+    }
+    {
+        KTimer t(h, CK_K_EMIT);
+        CKL(h) ck_rbs_index_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(h->d_rbs_open, h->d_rbs_openx, n, nf, h->d_rbs_fid, h->d_rbs_ffirst);
+        CKL(h) ck_rb_write_kernel<<<(n + 7) / 8, 256, 0, h->stream>>>(view_of(h), h->d_pubs, h->d_rbs_idx, n, h->d_pay_len, h->d_out_off, h->d_out,
+                                                                h->d_cols, h->n, h->d_rbs_recoff, codec ? h->d_rbs_plain : h->d_rbs_out,
+                                                                h->d_rbs_delta, h->d_rbs_fid, codec ? 0u : CK_RB_HEADER);
+        CKL(h) ck_rbs_layout_kernel<<<(nf + 256) / 256, 256, 0, h->stream>>>(h->d_rbs_ffirst, h->d_rbs_recoff, nf, codec, h->d_rbs_nch, h->d_rbs_foff);
+        CUDA_TRY(h, cudaGetLastError());
+    }
+    uint64_t total = plain + (uint64_t)CK_RB_HEADER * nf;
+    if (codec) {
+        if (run_scan(h, h->d_rbs_nch, nf, h->d_rbs_cbase, 0, h->d_rbs_tile, gr + 2)) return 1;
+        {
+            KTimer t(h, CK_K_CODEC);
+            CKL(h) ck_rbs_compress_kernel<<<h->rbs_pool / 128, 128, 0, h->stream>>>(h->d_rbs_plain, h->d_rbs_recoff, h->d_rbs_ffirst, h->d_rbs_cbase, nf,
+                gr + 2, (u32)cmax, codec, h->d_rbs_slots, h->d_rbs_csz, h->d_rbs_ccrc, h->d_rbs_tabs, h->d_rbs_dtabs);
+            CUDA_TRY(h, cudaGetLastError());
+        }
+        if (run_scan(h, h->d_rbs_csz, (u32)cmax, h->d_rbs_coff, 0, h->d_rbs_tile, gr + 3)) return 1;
+        {
+            KTimer t(h, CK_K_EMIT);
+            CKL(h) ck_rbs_fsize_kernel<<<(nf + 255) / 256, 256, 0, h->stream>>>(h->d_rbs_cbase, h->d_rbs_coff, nf, codec, h->d_rbs_fsize);
+            CUDA_TRY(h, cudaGetLastError());
+        }
+        if (run_scan(h, h->d_rbs_fsize, nf, h->d_rbs_foff, 0, h->d_rbs_tile, gr + 3)) return 1;
+        CUDA_TRY(h, cudaMemcpyAsync(h->h_rbs + 3, gr + 3, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+        total = h->h_rbs[3];
+        if (total > h->rbs_out_cap) {
+            snprintf(msg, sizeof msg, "ck_encode_recordbatches: %llu bytes of frames exceed the frame buffer (%llu bytes)",
+                     (unsigned long long)total, (unsigned long long)h->rbs_out_cap);
+            return fail(h, msg);
+        }
+    }
+    {
+        KTimer t(h, CK_K_EMIT);
+        if (codec) CKL(h) ck_rbs_copy_kernel<<<(u32)((cmax + 7) / 8), 256, 0, h->stream>>>(h->d_rbs_slots, h->d_rbs_recoff, h->d_rbs_ffirst, h->d_rbs_cbase,
+                                                                                        h->d_rbs_coff, nf, gr + 2, codec, h->d_rbs_foff, h->d_rbs_out);
+        CKL(h) ck_rbs_header_kernel<<<(nf + 127) / 128, 128, 0, h->stream>>>(h->d_rbs_out, h->d_rbs_foff, h->d_rbs_ffirst, h->d_rbs_recoff, nf, h->d_rbs_goff,
+                                                                           n_groups, host_base_offsets ? h->d_rbs_base : nullptr, timestamp_ms, codec,
+                                                                           h->d_rbs_cbase, h->d_rbs_ccrc, h->d_rbs_fgroup);
+        CKL(h) ck_rbs_crc_kernel<<<(nf + 7) / 8, 256, 0, h->stream>>>(h->d_rbs_out, h->d_rbs_foff, nf);
+        CUDA_TRY(h, cudaGetLastError());
+    }
+    h->rbs_nf = nf; h->rbs_total = total;
+    if (n_frames) *n_frames = nf;
+    if (total_bytes) *total_bytes = total;
+    return 0;
+}
+
+// the result of the last ck_encode_recordbatches: host_out[0 .. total_bytes) = the frames back to back,
+// host_frame_off[n_frames + 1], host_frame_group[n_frames]
+extern "C" int ck_fetch_recordbatches(ck_handle* h, uint8_t* host_out, uint64_t cap, uint64_t* host_frame_off, uint32_t* host_frame_group) {
+    cudaSetDevice(h->device);
+    if (h->rbs_total > cap) return fail(h, "ck_fetch_recordbatches: host buffer too small");
+    if (!h->rbs_nf) { if (host_frame_off) host_frame_off[0] = 0; return 0; }
+    CUDA_TRY(h, cudaMemcpyAsync(host_out, h->d_rbs_out, h->rbs_total, cudaMemcpyDeviceToHost, h->stream));
+    if (host_frame_off) CUDA_TRY(h, cudaMemcpyAsync(host_frame_off, h->d_rbs_foff, sizeof(long long) * (h->rbs_nf + 1), cudaMemcpyDeviceToHost, h->stream));
+    if (host_frame_group) CUDA_TRY(h, cudaMemcpyAsync(host_frame_group, h->d_rbs_fgroup, sizeof(u32) * h->rbs_nf, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     return 0;
 }
 

@@ -20,6 +20,13 @@
 //   (scan)               -> byte offset of every record inside the frame
 //   ck_rb_write_kernel   warp per record: varint header, key, value, the two headers calfkit's publishes carry
 //   ck_rb_header_kernel + ck_rb_crc_chunks/fold: the 61-byte batch header, CRC32C over the frame in 16 KB chunks
+// encode runs (produce, every topic-partition of a step; codec 0 none, 1 gzip, 3 LZ4):
+//   ck_rbs_split_kernel      warp per group: greedy split to max_bytes with exact in-frame sizes -> offsetDelta, size, opens
+//   (scans) + ck_rbs_index_kernel / ck_rbs_layout_kernel: record offsets, frame of every record, 64 KB chunks per frame
+//   ck_rb_write_kernel       the records, straight into the frames (codec 0) or into a plaintext scratch
+//   ck_rbs_compress_kernel   thread per 64 KB chunk (ck_lz4_enc.cuh / ck_deflate.cuh) into a slot of worst-case size
+//   (scans) + ck_rbs_copy_kernel / ck_rbs_header_kernel / ck_rbs_crc_kernel: assembly, headers, gzip CRC-32 fold, CRC32C
+// Worst-case section for P bytes of records: LZ4 11 + P + 4 ceil(P / 64 KB), gzip 20 + P + 10 ceil(P / 64 KB).
 #ifndef CK_KAFKA_CUH
 #define CK_KAFKA_CUH
 
@@ -77,26 +84,29 @@ CK_HD u32 ck_crc_span(const u32* __restrict__ t, const u8* __restrict__ p, u32 n
 
 #include "ck_inflate.cuh"
 #include "ck_lz4.cuh"
+#include "ck_deflate.cuh"
 
 #if defined(__CUDACC__)
-// a(x) * b(x) mod P(x), reflected representation (bit 31 = x^0)
-__device__ __forceinline__ u32 ck_gf_mul(u32 a, u32 b) {
+// a(x) * b(x) mod P(x), reflected representation (bit 31 = x^0); poly: the reflected polynomial, as for ck_crc_tables
+__device__ __forceinline__ u32 ck_gf_mul(u32 a, u32 b, u32 poly = CK_CRC_POLY) {
     u32 p = 0;
 #pragma unroll 4
     for (u32 m = 0x80000000u; m; m >>= 1) {
         if (a & m) p ^= b;
-        b = (b & 1u) ? (b >> 1) ^ CK_CRC_POLY : b >> 1;
+        b = (b & 1u) ? (b >> 1) ^ poly : b >> 1;
     }
     return p;
 }
 // x^(8 n) mod P
-__device__ __forceinline__ u32 ck_gf_xpow8(unsigned long long n) {
+__device__ __forceinline__ u32 ck_gf_xpow8(unsigned long long n, u32 poly = CK_CRC_POLY) {
     u32 p = 0x80000000u;                       // x^0
     u32 sq = 0x00800000u;                      // x^8
-    while (n) { if (n & 1ull) p = ck_gf_mul(sq, p); sq = ck_gf_mul(sq, sq); n >>= 1; }
+    while (n) { if (n & 1ull) p = ck_gf_mul(sq, p, poly); sq = ck_gf_mul(sq, sq, poly); n >>= 1; }
     return p;
 }
-__device__ __forceinline__ u32 ck_crc_combine(u32 crc_a, u32 crc_b, u32 xpow_len_b) { return ck_gf_mul(xpow_len_b, crc_a) ^ crc_b; }
+__device__ __forceinline__ u32 ck_crc_combine(u32 crc_a, u32 crc_b, u32 xpow_len_b, u32 poly = CK_CRC_POLY) {
+    return ck_gf_mul(xpow_len_b, crc_a, poly) ^ crc_b;
+}
 
 // CRC32C of one span by one warp (all lanes return it): lane 0 takes the odd-sized head so that every other lane holds
 // exactly `chunk` bytes and the tree fold shifts by multiples of one precomputed power
@@ -319,24 +329,28 @@ ck_rb_size_kernel(const ck_pub* __restrict__ pubs, const u32* __restrict__ idx, 
 }
 
 // warp per record; corr bytes are the raw JSON string content of deps.correlation_id (ids without escapes: the hashing
-// rule of ck_murmur2_key applies to escaped ones — those are rejected here by the host side before encoding)
+// rule of ck_murmur2_key applies to escaped ones — those are rejected here by the host side before encoding).
+// Record k goes to frame + hdr * (fid[k] + 1) + rec_off[k] with offsetDelta delta[k]; fid / delta = nullptr: one frame
+// (record k at frame + hdr + rec_off[k], offsetDelta k).  hdr = 0 writes bare records sections back to back.
 __global__ void __launch_bounds__(256)
 ck_rb_write_kernel(ck_view vw, const ck_pub* __restrict__ pubs, const u32* __restrict__ idx, u32 n, const u32* __restrict__ pay_len,
                    const long long* __restrict__ out_off, const u8* __restrict__ out, const u32* __restrict__ cols, u32 stride,
-                   const long long* __restrict__ rec_off, u8* __restrict__ frame) {
+                   const long long* __restrict__ rec_off, u8* __restrict__ frame, const u32* __restrict__ delta = nullptr,
+                   const u32* __restrict__ fid = nullptr, u32 hdr = CK_RB_HEADER) {
     u32 k = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (k >= n) return;
     ck_pub p = pubs[idx[k]];
     u32 rl; const u8* rec = ck_rec(vw, p.record, rl);
     u32 co = cols[(size_t)CK_COL_CORR_OFF * stride + p.record], cl = cols[(size_t)CK_COL_CORR_LEN * stride + p.record];
-    ck_rb_rec r = ck_rb_measure(k, pay_len[p.payload], cl, p.has_key != 0);
-    u8* d = frame + CK_RB_HEADER + rec_off[k];
+    u32 od = delta ? delta[k] : k;
+    ck_rb_rec r = ck_rb_measure(od, pay_len[p.payload], cl, p.has_key != 0);
+    u8* d = frame + (unsigned long long)hdr * (fid ? fid[k] + 1ull : 1ull) + rec_off[k];
     u32 pos = 0, vpos = 0, kpos = 0, cpos = 0;
     // every lane computes the same layout; lane 0 writes the small pieces, the warp copies key / value / header value
     u8 tmp[10];
     u32 m = ck_put_varint(tmp, r.body_len); if (lane == 0) for (u32 b = 0; b < m; b++) d[pos + b] = tmp[b]; pos += m;
     if (lane == 0) { d[pos] = 0; d[pos + 1] = 0; } pos += 2;                                  // attributes, timestampDelta = 0
-    m = ck_put_varint(tmp, k); if (lane == 0) for (u32 b = 0; b < m; b++) d[pos + b] = tmp[b]; pos += m;
+    m = ck_put_varint(tmp, od); if (lane == 0) for (u32 b = 0; b < m; b++) d[pos + b] = tmp[b]; pos += m;
     if (p.has_key) { m = ck_put_varint(tmp, cl); if (lane == 0) for (u32 b = 0; b < m; b++) d[pos + b] = tmp[b]; pos += m; kpos = pos; pos += cl; }
     else { if (lane == 0) d[pos] = 1; pos += 1; }                                             // zig-zag(-1) = null key
     m = ck_put_varint(tmp, r.val_len); if (lane == 0) for (u32 b = 0; b < m; b++) d[pos + b] = tmp[b]; pos += m; vpos = pos; pos += r.val_len;
@@ -399,6 +413,188 @@ __global__ void ck_rb_crc_fold_kernel(u8* __restrict__ frame, const long long* _
         c = ck_crc_combine(c, partial[k], len == CK_RB_CRC_CHUNK ? xp : ck_gf_xpow8(len));
     }
     ck_put_be32(frame + 17, c);
+}
+
+// ---- encode: runs of frames, compressed or not (ck_encode_recordbatches) ------------------------------------------------
+// Records of group g = idx[group_off[g] .. group_off[g+1]) (one topic-partition each) become a run of frames: a frame takes
+// the group's next records while 61 + their encoded sizes <= max_bytes, and always at least one.  offsetDelta is the
+// position inside the frame, so a record's size depends on where its frame starts: the split measures exact sizes.
+__device__ __forceinline__ u32 ck_rbs_size(const ck_pub* __restrict__ pubs, const u32* __restrict__ idx, u32 k, u32 d,
+                                           const u32* __restrict__ pay_len, const u32* __restrict__ cols, u32 stride) {
+    ck_pub p = pubs[idx[k]];
+    ck_rb_rec r = ck_rb_measure(d, pay_len[p.payload], cols[(size_t)CK_COL_CORR_LEN * stride + p.record], p.has_key != 0);
+    return ck_varint_size(r.body_len) + r.body_len;
+}
+
+// warp per group, 32 records per step: sizes at the open frame's positions, a prefix sum, one ballot for the first record
+// that does not fit.  Writes per record its offsetDelta, its size and whether it opens a frame.
+__global__ void __launch_bounds__(256)
+ck_rbs_split_kernel(const ck_pub* __restrict__ pubs, const u32* __restrict__ idx, const u32* __restrict__ group_off, u32 n_groups,
+                    const u32* __restrict__ pay_len, const u32* __restrict__ cols, u32 stride, u32 max_bytes,
+                    u32* __restrict__ delta, u32* __restrict__ sizes, u32* __restrict__ opens) {
+    u32 g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (g >= n_groups) return;
+    u32 end = group_off[g + 1], s = group_off[g], pos = s;             // s: first record of the open frame
+    unsigned long long acc = CK_RB_HEADER;
+    while (pos < end) {
+        u32 k = pos + lane;
+        unsigned long long inc = k < end ? ck_rbs_size(pubs, idx, k, k - s, pay_len, cols, stride) : 0ull;
+        u32 sz = (u32)inc;
+#pragma unroll
+        for (u32 o = 1; o < 32; o <<= 1) { unsigned long long t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
+        u32 over = __ballot_sync(0xffffffffu, k < end && acc + inc > max_bytes);
+        u32 take = over ? __ffs(over) - 1 : min(32u, end - pos);
+        if (take == 0 && pos == s) take = 1;                            // a record larger than the limit: a frame of its own
+        if (lane < take) { delta[k] = k - s; sizes[k] = sz; opens[k] = k == s; }
+        acc += take ? __shfl_sync(0xffffffffu, inc, take - 1) : 0ull;
+        pos += take;
+        if (over) { s = pos; acc = CK_RB_HEADER; }                      // the frame is full: the next one opens at pos
+    }
+}
+
+// thread per record: its frame (opens_x = exclusive scan of opens), and the first record of every frame
+__global__ void __launch_bounds__(256)
+ck_rbs_index_kernel(const u32* __restrict__ opens, const long long* __restrict__ opens_x, u32 n, u32 nf, u32* __restrict__ fid,
+                    u32* __restrict__ frame_first) {
+    u32 k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k == 0) frame_first[nf] = n;
+    if (k >= n) return;
+    u32 f = (u32)opens_x[k] + opens[k] - 1;
+    fid[k] = f;
+    if (opens[k]) frame_first[f] = k;
+}
+
+// thread per frame: records section size and 64 KB chunk count; uncompressed frames also get their place in the output
+// (frame_off[nf] = total), since their size is known here
+#define CK_RBS_CHUNK 65536u
+__global__ void __launch_bounds__(256)
+ck_rbs_layout_kernel(const u32* __restrict__ frame_first, const long long* __restrict__ rec_off, u32 nf, u32 codec,
+                     u32* __restrict__ nchunks, long long* __restrict__ frame_off) {
+    u32 f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f > nf) return;
+    long long s0 = rec_off[frame_first[f]];
+    if (!codec) { frame_off[f] = s0 + (long long)CK_RB_HEADER * f; return; }
+    if (f == nf) return;
+    long long sec = rec_off[frame_first[f + 1]] - s0;
+    nchunks[f] = (u32)((sec + CK_RBS_CHUNK - 1) / CK_RBS_CHUNK);
+}
+
+// the frame of chunk c: the last f with chunk_base[f] <= c
+__device__ __forceinline__ u32 ck_rbs_frame_of(const long long* __restrict__ base, u32 nf, unsigned long long c) {
+    u32 lo = 0, hi = nf;                                               // base[lo] <= c < base[hi]
+    while (hi - lo > 1) { u32 mid = (lo + hi) >> 1; if ((unsigned long long)base[mid] <= c) lo = mid; else hi = mid; }
+    return lo;
+}
+
+// one thread per chunk, grid-stride over a fixed pool of threads (each owns a hash table and DEFLATE scratch): chunk c of
+// frame f is plain[start, end) with start = the frame's section start + 64 KB * (c - chunk_base[f]).  Its compressed form
+// goes to the slot plain-offset + 64 * c of `slots` (never larger than the chunk + 64 bytes), its size to csz[c], and for
+// gzip its CRC-32 to ccrc[c].  Chunks c in [*n_chunks, cmax) get size 0 (the scan after this runs over the host's bound).
+__global__ void __launch_bounds__(128)
+ck_rbs_compress_kernel(const u8* __restrict__ plain, const long long* __restrict__ rec_off, const u32* __restrict__ frame_first,
+                       const long long* __restrict__ chunk_base, u32 nf, const unsigned long long* __restrict__ n_chunks, u32 cmax,
+                       u32 codec, u8* __restrict__ slots, u32* __restrict__ csz, u32* __restrict__ ccrc, u32* __restrict__ tabs,
+                       ck_dfl_tables* __restrict__ dtabs) {
+    __shared__ u32 t[1024];
+    ck_crc_tables(t, CK_CRC32_POLY);
+    u32 tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
+    unsigned long long nc = *n_chunks;
+    u32* tab = tabs + ((size_t)tid << CK_DFL_TAB_BITS);
+    for (u32 c = tid; c < cmax; c += nt) {
+        if (c >= nc) { csz[c] = 0; continue; }
+        u32 f = ck_rbs_frame_of(chunk_base, nf, c);
+        long long s0 = rec_off[frame_first[f]], s1 = rec_off[frame_first[f + 1]];
+        long long start = s0 + (long long)(c - chunk_base[f]) * CK_RBS_CHUNK;
+        u32 n = (u32)min((long long)CK_RBS_CHUNK, s1 - start);
+        u8* dst = slots + start + 64ll * c;
+        if (codec == CK_RB_LZ4) {
+            csz[c] = ck_lz4_enc_block(plain + start, n, dst, tab);
+        } else {
+            long long lo = start - s0 > 32768 ? start - 32768 : s0;    // history: up to 32 KB of the same section
+            csz[c] = ck_deflate_chunk(plain + lo, (u32)(start - lo), (u32)(start - lo) + n, dst, tab, dtabs[tid]);
+            ccrc[c] = ck_crc_span(t, plain + start, n);
+        }
+    }
+}
+
+// thread per frame: compressed frame size = header + codec header + its chunks + codec trailer
+__global__ void __launch_bounds__(256)
+ck_rbs_fsize_kernel(const long long* __restrict__ chunk_base, const long long* __restrict__ chunk_off, u32 nf, u32 codec,
+                    u32* __restrict__ fsize) {
+    u32 f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= nf) return;
+    long long cs = chunk_off[chunk_base[f + 1]] - chunk_off[chunk_base[f]];
+    fsize[f] = CK_RB_HEADER + (u32)cs + (codec == CK_RB_LZ4 ? CK_LZ4_HEAD + CK_LZ4_TAIL : CK_GZ_HEAD + CK_GZ_TAIL);
+}
+
+// warp per chunk: slot -> its place in the frame
+__global__ void __launch_bounds__(256)
+ck_rbs_copy_kernel(const u8* __restrict__ slots, const long long* __restrict__ rec_off, const u32* __restrict__ frame_first,
+                   const long long* __restrict__ chunk_base, const long long* __restrict__ chunk_off, u32 nf,
+                   const unsigned long long* __restrict__ n_chunks, u32 codec, const long long* __restrict__ frame_off, u8* __restrict__ out) {
+    unsigned long long c = (blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x) >> 5;
+    u32 lane = threadIdx.x & 31;
+    if (c >= *n_chunks) return;
+    u32 f = ck_rbs_frame_of(chunk_base, nf, c);
+    long long start = rec_off[frame_first[f]] + (long long)(c - chunk_base[f]) * CK_RBS_CHUNK;
+    u32 head = codec == CK_RB_LZ4 ? CK_LZ4_HEAD : CK_GZ_HEAD;
+    u8* dst = out + frame_off[f] + CK_RB_HEADER + head + (chunk_off[c] - chunk_off[chunk_base[f]]);
+    ck_warp_copy(dst, slots + start + 64ll * c, (u32)(chunk_off[c + 1] - chunk_off[c]), lane);
+}
+
+// thread per frame: the 61-byte header (everything but the CRC32C), the codec's header and trailer (gzip: CRC-32 of the
+// section folded from the per-chunk CRCs), and the frame's group.  Frame f of group g: baseOffset = base_offsets[g] +
+// the records of g in earlier frames.
+__global__ void __launch_bounds__(128)
+ck_rbs_header_kernel(u8* __restrict__ out, const long long* __restrict__ frame_off, const u32* __restrict__ frame_first,
+                     const long long* __restrict__ rec_off, u32 nf, const u32* __restrict__ group_off, u32 n_groups,
+                     const long long* __restrict__ base_offsets, long long timestamp_ms, u32 codec,
+                     const long long* __restrict__ chunk_base, const u32* __restrict__ ccrc, u32* __restrict__ frame_group) {
+    u32 f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= nf) return;
+    u32 k0 = frame_first[f], cnt = frame_first[f + 1] - k0;
+    u32 lo = 0, hi = n_groups;                                         // the group holding k0: last g with group_off[g] <= k0
+    while (hi - lo > 1) { u32 mid = (lo + hi) >> 1; if (group_off[mid] <= k0) lo = mid; else hi = mid; }
+    u8* fr = out + frame_off[f];
+    unsigned long long flen = (unsigned long long)(frame_off[f + 1] - frame_off[f]);
+    ck_put_be64(fr, (unsigned long long)((base_offsets ? base_offsets[lo] : 0ll) + (k0 - group_off[lo])));
+    ck_put_be32(fr + 8, (u32)(flen - 12));
+    ck_put_be32(fr + 12, 0);                                 // partitionLeaderEpoch
+    fr[16] = 2;
+    fr[21] = 0; fr[22] = (u8)codec;                          // attributes: codec, CreateTime
+    ck_put_be32(fr + 23, cnt - 1);                           // lastOffsetDelta
+    ck_put_be64(fr + 27, (unsigned long long)timestamp_ms);
+    ck_put_be64(fr + 35, (unsigned long long)timestamp_ms);
+    ck_put_be64(fr + 43, ~0ull);                             // producerId -1
+    fr[51] = 0xff; fr[52] = 0xff;                            // producerEpoch -1
+    ck_put_be32(fr + 53, 0xffffffffu);                       // baseSequence -1
+    ck_put_be32(fr + 57, cnt);
+    frame_group[f] = lo;
+    if (codec == CK_RB_LZ4) {
+        ck_lz4_frame_head(fr + CK_RB_HEADER);
+        ck_put_be32(fr + flen - CK_LZ4_TAIL, 0);             // EndMark
+    } else if (codec == CK_RB_GZIP) {
+        long long s0 = rec_off[k0], sec = rec_off[frame_first[f + 1]] - s0;
+        u32 crc = 0, xfull = ck_gf_xpow8(CK_RBS_CHUNK, CK_CRC32_POLY);
+        for (long long c = chunk_base[f]; c < chunk_base[f + 1]; c++) {
+            long long len = min((long long)CK_RBS_CHUNK, sec - (c - chunk_base[f]) * (long long)CK_RBS_CHUNK);
+            crc = ck_crc_combine(crc, ccrc[c], len == CK_RBS_CHUNK ? xfull : ck_gf_xpow8((unsigned long long)len, CK_CRC32_POLY), CK_CRC32_POLY);
+        }
+        ck_gzip_head(fr + CK_RB_HEADER);
+        ck_gzip_tail(fr + flen - CK_GZ_TAIL, crc, (u32)sec);
+    }
+}
+
+// warp per frame: CRC32C of the covered bytes [21, end) of every frame
+__global__ void __launch_bounds__(256)
+ck_rbs_crc_kernel(u8* __restrict__ out, const long long* __restrict__ frame_off, u32 nf) {
+    __shared__ u32 t[1024];
+    ck_crc_tables(t);
+    u32 w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (w >= nf) return;
+    u8* fr = out + frame_off[w];
+    u32 c = ck_crc32c_warp(t, fr + CK_RB_CRC_FROM, (u32)(frame_off[w + 1] - frame_off[w]) - CK_RB_CRC_FROM, lane);
+    if (lane == 0) ck_put_be32(fr + 17, c);
 }
 
 #endif  // __CUDACC__

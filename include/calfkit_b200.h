@@ -102,6 +102,26 @@ int  ck_fetch_rb_index(ck_handle* h, int64_t* val_off, uint32_t* val_len, int64_
 int  ck_fetch_rb_decompressed(ck_handle* h, uint8_t* host_dst, uint64_t cap, uint64_t* base, uint64_t* len);
 int  ck_encode_recordbatch(ck_handle* h, const uint32_t* host_idx, uint32_t n, int64_t base_offset, int64_t timestamp_ms,
                            uint8_t* host_frame, uint64_t cap, uint64_t* frame_len);
+/* ck_encode_recordbatches: publishes host_idx[0..n) of the current plan (indices of live publishes), in groups: group g =
+ * host_idx[group_off[g] .. group_off[g+1]), one topic-partition each, in send order.  Every group becomes a run of v2
+ * frames, as a producer that closes a batch at max_batch_bytes writes them: a frame takes the group's next records while
+ * 61 + (their encoded sizes) <= max_batch_bytes, and always at least one; frames never span groups; offsetDelta is the
+ * position inside the frame.  codec: 0 none, 1 gzip, 3 LZ4 (anything else is an error); base_offsets: NULL = 0 for every
+ * group; frame k of group g gets baseOffset = base_offsets[g] + (records of g in earlier frames).  Compressed sections are
+ * made on the device in 64 KB chunks:
+ *   LZ4   one LZ4 frame, descriptor 60 40 82 (independent 64 KB blocks, no checksums, no content size); a chunk that does
+ *         not get smaller is stored raw.  Section <= 11 + P + 4 * ceil(P / 65536) bytes for P bytes of records.
+ *   gzip  one member, header 1f 8b 08 00 00000000 00 ff; every chunk one non-final dynamic-Huffman block + an empty stored
+ *         block (or stored blocks when smaller), matches up to 32 KB back into the previous chunk; final block 03 00,
+ *         CRC-32, ISIZE.  Section <= 20 + P + 10 * ceil(P / 65536) bytes.
+ * The output depends on the arguments only.  *n_frames / *total_bytes describe the result, which stays on the device
+ * until ck_fetch_recordbatches; a request larger than the scratch (sized from max_out_bytes / max_payloads) fails.
+ * ck_fetch_recordbatches: host_out[0 .. total_bytes) = the frames back to back, frame_off[n_frames + 1],
+ * frame_group[n_frames]. */
+int  ck_encode_recordbatches(ck_handle* h, const uint32_t* host_idx, uint32_t n, const uint32_t* host_group_off,
+                             uint32_t n_groups, const int64_t* host_base_offsets, int64_t timestamp_ms, uint32_t codec,
+                             uint32_t max_batch_bytes, uint32_t* n_frames, uint64_t* total_bytes);
+int  ck_fetch_recordbatches(ck_handle* h, uint8_t* host_out, uint64_t cap, uint64_t* host_frame_off, uint32_t* host_frame_group);
 
 /* tool node, host tools only: gather every record's tool-call `args` JSON into the output buffer
  * (payload i = args of record i, empty when the record does not reach the tool). */
